@@ -1,8 +1,9 @@
 """FLAC ingest (SURVEY 8f row 3a): csrc/flac.cu through the C ABI and audio.decode_flac -- host code, runs without a GPU.
 
-Goldens: the PCM MD5s of the reference's fixtures client/{3sec,10sec,30sec}.flac (SURVEY.md section 4, parsed from
-their STREAMINFO) when /root/reference is present, plus streams made by tests/flac_writer.py for every decoder path
-the libFLAC-made mono fixtures do not reach."""
+Goldens: the PCM MD5s of the reference's libFLAC-made fixtures (SURVEY.md section 4, parsed from their STREAMINFO):
+client/3sec.flac as it is, and the first 10 frames of client/{10sec,30sec}.flac (tests/golden/client_*_head.flac, cut by
+scripts/gen_golden_flac.py; the MD5 of the full 10 s / 30 s recordings is c5b99673... / 3a541ad6...), plus streams made
+by tests/flac_writer.py for every decoder path the libFLAC-made mono fixtures do not reach."""
 import hashlib
 import os
 
@@ -12,19 +13,18 @@ import pytest
 from tests import flac_writer as fw
 from willow_inference_server_b200 import _lib, audio
 
-REF = "/root/reference/client"
 FIXTURES = [("3sec.flac", 61440, "ad790df21d4d9d223d3f34227b5cfedd"),
-            ("10sec.flac", 171008, "c5b99673d012d9a8f5d19dd68874a121"),
-            ("30sec.flac", 467968, "3a541ad6463fe6e884e5995212b518fa")]
+            ("10sec_head.flac", 40960, "b8310575537022d81af8341b0aa377ec"),
+            ("30sec_head.flac", 40960, "97c9c8e0886212e3deadeaf1e58e88a7")]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference fixtures are only present in the build container")
 @pytest.mark.parametrize("name,n,md5", FIXTURES)
-def test_reference_fixtures_decode_to_their_md5(name, n, md5):
-    pcm, sr = audio.decode_flac(os.path.join(REF, name))          # verify=True already checks STREAMINFO's MD5
+def test_reference_fixtures_decode_to_their_md5(name, n, md5, golden_dir):
+    path = os.path.join(golden_dir, "client_" + name)
+    pcm, sr = audio.decode_flac(path)                              # verify=True already checks STREAMINFO's MD5
     assert sr == 16000 and pcm.dtype == np.int16 and pcm.shape == (n,)
     assert hashlib.md5(pcm.astype("<i2").tobytes()).hexdigest() == md5
-    x = audio.load_audio(os.path.join(REF, name))
+    x = audio.load_audio(path)
     assert x.dtype == np.float32 and x.shape == (n,) and np.abs(x).max() <= 1.0
     assert np.array_equal(x, pcm.astype(np.float32) / 32768.0)
 
