@@ -71,6 +71,19 @@ int wisb_generate_ex(wisb_handle* h, const float* mel, int B, const int32_t* pro
                      const int32_t* extra_suppress, int n_extra, int32_t* out_ids, int out_stride, int32_t* out_len,
                      float* out_score);
 
+/* Same call with Whisper's timestamp rules, what CTranslate2 applies when the prompt lacks <|notimestamps|>
+ * (the reference's prompts keep that token, main.py:529, :661; removing it asks for timestamps).  Timestamp tokens are
+ * [no_timestamps + 1, n_vocab); the rules are those of openai-whisper's ApplyTimestampRules: <|notimestamps|> is never
+ * generated, timestamps come in pairs (except right before <|endoftext|>) and never decrease, the first generated token
+ * is a timestamp no later than no_timestamps + 1 + max_initial_timestamp_index, and when the timestamps' total
+ * probability beats every text token a timestamp is generated.  out_ids keep the timestamp tokens (<|endoftext|> is
+ * still left out).  Returns 1 when a prompt contains <|notimestamps|> or max_initial_timestamp_index is outside
+ * [0, n_vocab - no_timestamps - 2]. */
+int wisb_generate_ts(wisb_handle* h, const float* mel, int B, const int32_t* prompts, int prompt_len, int beam_size,
+                     float patience, float length_penalty, int max_length, const int32_t* max_length_per_utt,
+                     const int32_t* extra_suppress, int n_extra, int max_initial_timestamp_index, int32_t* out_ids,
+                     int out_stride, int32_t* out_len, float* out_score);
+
 /* (5) per utterance: language token ids sorted by probability (descending) and the probabilities.
  * lang_ids_out int32 [B, n_langs], probs_out float32 [B, n_langs]. */
 int wisb_detect_language(wisb_handle* h, const float* mel, int B, int32_t* lang_ids_out, float* probs_out);

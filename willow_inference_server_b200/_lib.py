@@ -34,6 +34,9 @@ _SIGS = {
                                 C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "wisb_generate_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_float,
                                    C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "wisb_generate_ts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_float,
+                                   C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
+                                   C.c_void_p]),
     "wisb_detect_language": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "wisb_get_timing": (C.c_int, [C.c_void_p, C.c_void_p]),
     "wisb_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int]),
@@ -163,7 +166,9 @@ class Handle:
         return out
 
     def generate(self, mel, prompts, beam_size=5, patience=1.0, length_penalty=1.0, max_length=448, extra_suppress=(),
-                 B=None):
+                 B=None, timestamps=False, max_initial_timestamp_index=50):
+        """-> (token ids per window, scores).  ``timestamps=True`` applies Whisper's timestamp rules (wisb_generate_ts):
+        the prompts must not contain <|notimestamps|>, and the ids keep the timestamp tokens."""
         prompts = np.ascontiguousarray(prompts, np.int32)
         if prompts.ndim != 2:
             raise ValueError("prompts must be [B, prompt_len]")
@@ -184,9 +189,16 @@ class Handle:
         lens = np.zeros(B, np.int32)
         scores = np.zeros(B, np.float32)
         extra = np.ascontiguousarray(list(extra_suppress), np.int32)
-        check(lib().wisb_generate_ex(self._h, ptr(mel), B, ptr(prompts), prompts.shape[1], int(beam_size), float(patience),
-                                     float(length_penalty), int(max_length), ptr(per_utt), ptr(extra) if extra.size else None,
-                                     extra.size, ptr(ids), stride, ptr(lens), ptr(scores)))
+        if timestamps:
+            check(lib().wisb_generate_ts(self._h, ptr(mel), B, ptr(prompts), prompts.shape[1], int(beam_size),
+                                         float(patience), float(length_penalty), int(max_length), ptr(per_utt),
+                                         ptr(extra) if extra.size else None, extra.size, int(max_initial_timestamp_index),
+                                         ptr(ids), stride, ptr(lens), ptr(scores)))
+        else:
+            check(lib().wisb_generate_ex(self._h, ptr(mel), B, ptr(prompts), prompts.shape[1], int(beam_size),
+                                         float(patience), float(length_penalty), int(max_length), ptr(per_utt),
+                                         ptr(extra) if extra.size else None, extra.size, ptr(ids), stride, ptr(lens),
+                                         ptr(scores)))
         return [ids[b, : lens[b]].tolist() for b in range(B)], scores.tolist()
 
     def detect_language(self, mel, B=None):

@@ -167,6 +167,11 @@ def transcribe_long(model, audio, prompt, tokenizer, *, beam_size: int = 5, batc
     Returns the merged token ids (numpy int array), ready for ``whisper_processor.decode``."""
     from .models import StorageView
 
+    # Timestamps are relative to their window: stitching them with the token-level LCS merge would give wrong times, so
+    # a prompt that asks for timestamps is refused (checked with the engine's ids, when it has them)
+    dims = getattr(model if model is not None else getattr(batcher, "_model", None), "dims", None)
+    if isinstance(dims, dict) and "no_timestamps" in dims and dims["no_timestamps"] not in list(prompt):
+        raise ValueError("transcribe_long does not decode timestamps: the prompt must contain <|notimestamps|>")
     pcm = np.asarray(audio)
     if pcm.ndim == 1 and pcm.shape[0] <= N_SAMPLES:
         # <= 30 s: the reference does not window at all (main.py:587-617), it decodes one zero-padded 30-s window

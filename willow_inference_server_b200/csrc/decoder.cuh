@@ -89,6 +89,9 @@ struct SearchArgs {
   int* row_pos = nullptr;         // [R] position fed by every row this step (batched pass); advanced with st->pos
   int* row_slot = nullptr;        // [R] cache slot every row writes this step's K/V to (= its own row)
   const int* max_new_u = nullptr; // optional [n_utt]: per-utterance cap on generated tokens (<= max_new)
+  // timestamp rules (search.cu): first timestamp token (<|notimestamps|> + 1), -1 = off; largest index of the first
+  // timestamp above ts_begin
+  int ts_begin = -1, max_init_ts = 0;
 };
 void search_step_run(const SearchArgs& a, cudaStream_t stream);
 // prompt prefill: no search, just feed the next prompt token and advance the position

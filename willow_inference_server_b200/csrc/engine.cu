@@ -78,7 +78,7 @@ struct DecLayerW {
 };
 
 struct GraphKey {
-  int n_utt, beam, prompt_len, max_new, max_hyp, u0, b_total, batched;
+  int n_utt, beam, prompt_len, max_new, max_hyp, u0, b_total, batched, ts_begin, max_init_ts;
   float lp;
   bool operator<(const GraphKey& o) const {
     return memcmp(this, &o, sizeof(GraphKey)) < 0;
@@ -658,6 +658,7 @@ struct DecodeCfg {
   int u0, n_utt, B_total, beam, prompt_len, max_new, max_hyp;
   float lp;
   int per_utt_max_new = 0;  // h->max_new_u holds a per-utterance cap (<= max_new)
+  int ts_begin = -1, max_init_ts = 0;  // timestamp rules (SearchArgs): first timestamp token, -1 = off
 };
 
 SearchArgs make_search_args(wisb_handle* h, const DecodeCfg& c) {
@@ -698,6 +699,8 @@ SearchArgs make_search_args(wisb_handle* h, const DecodeCfg& c) {
   a.row_pos = h->row_pos.p;
   a.row_slot = h->row_slot.p;
   a.max_new_u = c.per_utt_max_new ? h->max_new_u.p : nullptr;
+  a.ts_begin = c.ts_begin;
+  a.max_init_ts = c.max_init_ts;
   return a;
 }
 
@@ -905,6 +908,7 @@ DecGraphs& get_graphs(wisb_handle* h, const DecodeCfg& c) {
   key.n_utt = c.n_utt; key.beam = c.beam; key.prompt_len = c.prompt_len; key.max_new = c.max_new;
   key.max_hyp = c.max_hyp; key.lp = c.lp;
   key.u0 = c.u0; key.b_total = c.B_total;  // they move the cross-K/V base pointers baked into the graph
+  key.ts_begin = c.ts_begin; key.max_init_ts = c.max_init_ts;  // baked into the search kernels' arguments
   auto it = h->graphs.find(key);
   if (it != h->graphs.end()) return it->second;
   if (h->graphs.size() > 64) {  // bound the cache
@@ -1233,6 +1237,7 @@ int decode_batch(wisb_handle* h, const DecodeCfg& c, const int32_t* prompts, con
       key.n_utt = c.n_utt; key.beam = c.beam; key.prompt_len = c.prompt_len; key.max_new = c.max_new;
       key.max_hyp = c.max_hyp; key.lp = c.lp; key.u0 = c.u0; key.b_total = c.B_total;
       key.batched = 1 + c.per_utt_max_new;
+      key.ts_begin = c.ts_begin; key.max_init_ts = c.max_init_ts;
       auto it = h->graphs.find(key);
       if (it == h->graphs.end()) {
         if (h->graphs.size() > 64) drop_graphs(h);
@@ -1512,10 +1517,11 @@ int wisb_logmel(wisb_handle* h, const void* pcm, int pcm_dtype, int pcm_on_devic
   });
 }
 
-int wisb_generate_ex(wisb_handle* h, const float* mel, int B, const int32_t* prompts, int prompt_len, int beam_size,
-                     float patience, float length_penalty, int max_length, const int32_t* max_length_per_utt,
-                     const int32_t* extra_suppress, int n_extra, int32_t* out_ids, int out_stride, int32_t* out_len,
-                     float* out_score) {
+// wisb_generate_ex (timestamps == 0) and wisb_generate_ts (timestamps != 0)
+static int generate_common(wisb_handle* h, const float* mel, int B, const int32_t* prompts, int prompt_len, int beam_size,
+                           float patience, float length_penalty, int max_length, const int32_t* max_length_per_utt,
+                           const int32_t* extra_suppress, int n_extra, int timestamps, int max_initial_timestamp_index,
+                           int32_t* out_ids, int out_stride, int32_t* out_len, float* out_score) {
   return guarded(h, [&] {
     const Dims& dm = h->dims;
     WISB_REQUIRE(h->blob != nullptr, "handle has no model (created by wisb_create_frontend)");
@@ -1528,6 +1534,14 @@ int wisb_generate_ex(wisb_handle* h, const float* mel, int B, const int32_t* pro
     WISB_REQUIRE(n_extra >= 0 && (n_extra == 0 || extra_suppress != nullptr), "bad extra_suppress");
     for (long long i = 0; i < static_cast<long long>(B) * prompt_len; ++i)
       WISB_REQUIRE(prompts[i] >= 0 && prompts[i] < dm.n_vocab, "prompt token outside the vocabulary");
+    const int ts_begin = timestamps ? dm.no_timestamps + 1 : -1;
+    if (timestamps) {
+      WISB_REQUIRE(ts_begin > dm.eot && ts_begin < dm.n_vocab, "the model's vocabulary has no timestamp tokens");
+      WISB_REQUIRE(max_initial_timestamp_index >= 0 && max_initial_timestamp_index <= dm.n_vocab - ts_begin - 1,
+                   "max_initial_timestamp_index must be in [0, number of timestamp tokens - 1]");
+      for (long long i = 0; i < static_cast<long long>(B) * prompt_len; ++i)
+        WISB_REQUIRE(prompts[i] != dm.no_timestamps, "timestamp decoding: the prompt must not contain <|notimestamps|>");
+    }
     auto new_tokens = [&](int ml) {  // CTranslate2: at most max_length / 2 new tokens, max_length in total
       int v = ml / 2 < ml - prompt_len ? ml / 2 : ml - prompt_len;
       return v < 0 ? 0 : v;
@@ -1561,6 +1575,8 @@ int wisb_generate_ex(wisb_handle* h, const float* mel, int B, const int32_t* pro
     c.max_hyp = static_cast<int>(beam_size * patience + 0.5f);
     if (c.max_hyp < 1) c.max_hyp = 1;
     c.lp = length_penalty;
+    c.ts_begin = ts_begin;
+    c.max_init_ts = timestamps ? max_initial_timestamp_index : 0;
     // Utterances are encoded and decoded in groups that share every decoder pass: the group's rows (utterances x beams)
     // are the M dimension of the batched pass, so the decoder weights stream once per generated token for the whole
     // group.  The group size only bounds the workspaces (cross K/V: 252 MB per large-v2 utterance).
@@ -1616,6 +1632,23 @@ int wisb_generate_ex(wisb_handle* h, const float* mel, int B, const int32_t* pro
     h->timing[7] = static_cast<float>(h->launches);
     h->prof_collect();
   });
+}
+
+int wisb_generate_ex(wisb_handle* h, const float* mel, int B, const int32_t* prompts, int prompt_len, int beam_size,
+                     float patience, float length_penalty, int max_length, const int32_t* max_length_per_utt,
+                     const int32_t* extra_suppress, int n_extra, int32_t* out_ids, int out_stride, int32_t* out_len,
+                     float* out_score) {
+  return generate_common(h, mel, B, prompts, prompt_len, beam_size, patience, length_penalty, max_length,
+                         max_length_per_utt, extra_suppress, n_extra, 0, 0, out_ids, out_stride, out_len, out_score);
+}
+
+int wisb_generate_ts(wisb_handle* h, const float* mel, int B, const int32_t* prompts, int prompt_len, int beam_size,
+                     float patience, float length_penalty, int max_length, const int32_t* max_length_per_utt,
+                     const int32_t* extra_suppress, int n_extra, int max_initial_timestamp_index, int32_t* out_ids,
+                     int out_stride, int32_t* out_len, float* out_score) {
+  return generate_common(h, mel, B, prompts, prompt_len, beam_size, patience, length_penalty, max_length,
+                         max_length_per_utt, extra_suppress, n_extra, 1, max_initial_timestamp_index, out_ids, out_stride,
+                         out_len, out_score);
 }
 
 int wisb_generate(wisb_handle* h, const float* mel, int B, const int32_t* prompts, int prompt_len, int beam_size,

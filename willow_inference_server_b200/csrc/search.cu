@@ -5,6 +5,7 @@
 // /root/reference/main.py:687-692 with the library defaults patience=1, length_penalty=1, suppress_blank=True,
 // suppress_tokens=[-1], num_hypotheses=1):
 //   * processors: `suppress_ids` -> -inf every step; {blank, eot} -> -inf at the first generated step
+//   * timestamp rules when the prompt has no <|notimestamps|> (SearchArgs::ts_begin >= 0): see ts_rules below
 //   * scores: log_softmax(logits) + cumulative beam score, divided by (step+1)^length_penalty
 //   * candidates: top 2*beam of beam*V (ties: lowest flat index); at step 0 only beam 0 is live
 //   * the first `beam` candidates that end in eot (or any at the last step) become hypotheses and are replaced by the
@@ -72,7 +73,53 @@ __device__ void block_select(unsigned long long (&keys)[PER], int n_cand, unsign
 
 // grid (TOPK_CHUNKS, R): partial top-n_cand of one chunk of one row
 constexpr int TK_THREADS = 256;
-constexpr int TK_PER = 8;  // 256 * 8 = 2048 >= ceil(51865 / 32) = 1621
+constexpr int TK_PER = 8;  // 256 * 8 = 2048 >= ceil(51865 / 32) = 1621 (timestamp mode: ceil(50364 / 31) = 1625, 1501)
+
+// Timestamp mode (a.ts_begin >= 0): the rules of HF WhisperTimeStampLogitsProcessor (a port of openai-whisper's
+// ApplyTimestampRules) for row r at generation step `gen`, derived from the row's own generated tokens
+// seq[*flip][r][0, gen) -- already per beam and reordered by the bookkeeping, so no extra per-row state is carried.
+// The chunk layout changes too: the text tokens [0, ts_begin) are spread over chunks 0 .. TOPK_CHUNKS-2 and the
+// timestamps [ts_begin, n_vocab) form the last chunk alone, so that the merge finds the timestamps' (max, sum exp) and
+// the text maximum among the partials as they are (rule 5).  Outputs: the chunk [v0, v1) and the tokens of it the rules
+// let through, [lo, hi) minus `hole`.  Called by every thread of the block.
+__device__ void ts_rules(const SearchArgs& a, int r, int gen, int chunk, int& v0, int& v1, int& lo, int& hi, int& hole,
+                         int* s_i /*[TK_THREADS / 32]*/) {
+  const int tb = a.ts_begin;
+  const int* hist = a.seq[*a.flip] + static_cast<long long>(r) * a.max_new;
+  int li = -1;  // position of the last timestamp in the history
+  for (int t = threadIdx.x; t < gen; t += blockDim.x)
+    if (hist[t] >= tb) li = t;
+  li = __reduce_max_sync(0xffffffffu, li);
+  if ((threadIdx.x & 31) == 0) s_i[threadIdx.x >> 5] = li;
+  __syncthreads();
+  for (int w = 0; w < TK_THREADS / 32; ++w) li = max(li, s_i[w]);
+  const bool last_ts = gen >= 1 && hist[gen - 1] >= tb;
+  const bool pen_ts = gen < 2 || hist[gen - 2] >= tb;
+  int text_lo = 0, ts_lo = tb, ts_hi = a.n_vocab;
+  if (last_ts) {
+    if (pen_ts) ts_hi = tb;  // a pair was just completed (or the history is one timestamp): text next
+    else text_lo = a.eot;    // a segment was just closed: another timestamp or <|endoftext|> next
+  }
+  // timestamps never decrease; right after a segment closes the next one may open at the same time
+  if (li >= 0) ts_lo = max(ts_lo, hist[li] + ((last_ts && !pen_ts) ? 0 : 1));
+  if (gen == 0) {  // the first generated token is a timestamp no later than ts_begin + max_init_ts
+    text_lo = tb;
+    ts_hi = min(a.n_vocab, tb + a.max_init_ts + 1);
+  }
+  if (chunk == TOPK_CHUNKS - 1) {
+    v0 = tb;
+    v1 = a.n_vocab;
+    lo = ts_lo;
+    hi = ts_hi;
+  } else {
+    const int per = (tb + TOPK_CHUNKS - 2) / (TOPK_CHUNKS - 1);
+    v0 = chunk * per;
+    v1 = min(tb, v0 + per);
+    lo = text_lo;
+    hi = v1;
+    hole = tb - 1;  // <|notimestamps|> is never generated
+  }
+}
 
 __global__ void __launch_bounds__(TK_THREADS) topk_partial_kernel(const SearchArgs a) {
   // Within one row the ranking by processed logit equals the ranking by score, so the per-chunk stage needs no
@@ -80,13 +127,22 @@ __global__ void __launch_bounds__(TK_THREADS) topk_partial_kernel(const SearchAr
   // the row's lse and into scores.  (This replaced a separate two-pass lse kernel: 55 us -> 0.)
   __shared__ unsigned long long s_red[32];
   __shared__ float s_f[32];
+  __shared__ int s_i[TK_THREADS / 32];
   if (a.st->all_done) return;  // a step enqueued ahead of the host's poll
   const int chunk = blockIdx.x, r = blockIdx.y;
-  const bool first = a.st->gen_step == 0;
+  const int gen = a.st->gen_step;
+  const bool first = gen == 0;
   const float* row = a.logits + static_cast<long long>(r) * a.ldl;
-  const int per_chunk = (a.n_vocab + TOPK_CHUNKS - 1) / TOPK_CHUNKS;
-  const int v0 = chunk * per_chunk;
-  const int v1 = min(a.n_vocab, v0 + per_chunk);
+  int v0, v1, lo, hi, hole = -1;
+  if (a.ts_begin < 0) {
+    const int per_chunk = (a.n_vocab + TOPK_CHUNKS - 1) / TOPK_CHUNKS;
+    v0 = chunk * per_chunk;
+    v1 = min(a.n_vocab, v0 + per_chunk);
+    lo = v0;
+    hi = v1;
+  } else {
+    ts_rules(a, r, gen, chunk, v0, v1, lo, hi, hole, s_i);
+  }
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   unsigned long long keys[TK_PER];
   float lg[TK_PER];
@@ -97,7 +153,7 @@ __global__ void __launch_bounds__(TK_THREADS) topk_partial_kernel(const SearchAr
     keys[i] = 0ull;
     lg[i] = -INFINITY;
     if (v < v1) {
-      lg[i] = masked_logit(a, row, v, first);
+      lg[i] = (v < lo || v >= hi || v == hole) ? -INFINITY : masked_logit(a, row, v, first);
       if (lg[i] != -INFINITY) keys[i] = pack_key(lg[i], static_cast<unsigned>(v));
       mx = fmaxf(mx, lg[i]);
     }
@@ -127,7 +183,8 @@ __global__ void __launch_bounds__(TK_THREADS) topk_partial_kernel(const SearchAr
 // grid (n_utt): merge beam * TOPK_CHUNKS * n_cand partial keys -> sorted candidate list
 constexpr int TM_PER = (MAX_BEAM * TOPK_CHUNKS * MAX_CAND + TK_THREADS - 1) / TK_THREADS;  // 16
 
-__device__ __forceinline__ void topk_merge_body(const SearchArgs& a, unsigned long long* s_red, unsigned long long* s_out, float* s_lse) {
+__device__ __forceinline__ void topk_merge_body(const SearchArgs& a, unsigned long long* s_red, unsigned long long* s_out, float* s_lse,
+                                                int* s_ts_only) {
   const int u = blockIdx.x;
   const int gen = a.st->gen_step;
   const bool first = gen == 0;
@@ -141,8 +198,24 @@ __device__ __forceinline__ void topk_merge_body(const SearchArgs& a, unsigned lo
       const float pm = a.part_max[r * TOPK_CHUNKS + c];
       if (pm != -INFINITY) t += a.part_sum[r * TOPK_CHUNKS + c] * __expf(pm - mx);
     }
-    s_lse[threadIdx.x] = mx + logf(t);
-    a.row_lse[r] = s_lse[threadIdx.x];
+    float lse = mx + logf(t);
+    int ts_only = 0;
+    if (a.ts_begin >= 0) {
+      // timestamp rule 5: when the timestamps' total probability beats every single text token, text is banned and the
+      // row is renormalised over the timestamps (the last chunk holds exactly them; the log-softmax shift cancels)
+      const int cts = TOPK_CHUNKS - 1;
+      float mtext = -INFINITY;
+      for (int c = 0; c < cts; ++c) mtext = fmaxf(mtext, a.part_max[r * TOPK_CHUNKS + c]);
+      const float pm = a.part_max[r * TOPK_CHUNKS + cts];
+      const float lse_ts = pm == -INFINITY ? -INFINITY : pm + logf(a.part_sum[r * TOPK_CHUNKS + cts]);
+      if (lse_ts > mtext) {
+        lse = lse_ts;
+        ts_only = 1;
+      }
+    }
+    s_lse[threadIdx.x] = lse;
+    s_ts_only[threadIdx.x] = ts_only;
+    a.row_lse[r] = lse;
   }
   __syncthreads();
   const int total = a.beam * TOPK_CHUNKS * a.n_cand;
@@ -157,7 +230,7 @@ __device__ __forceinline__ void topk_merge_body(const SearchArgs& a, unsigned lo
       const int k = rc / TOPK_CHUNKS;    // beam index
       const unsigned long long pk = a.part[(static_cast<long long>(u * a.beam) * TOPK_CHUNKS + rc) * MAX_CAND + c];
       // at the first step every beam holds the same prefix: only beam 0 counts
-      if (pk != 0ull && !(first && k > 0)) {
+      if (pk != 0ull && !(first && k > 0) && !(s_ts_only[k] && rc % TOPK_CHUNKS != TOPK_CHUNKS - 1)) {
         const float lg = ord2f(static_cast<unsigned>(pk >> 32));
         const unsigned v = ~static_cast<unsigned>(pk & 0xffffffffull);
         const float sc = ((lg - s_lse[k]) + a.cum[u * a.beam + k]) / norm;
@@ -277,12 +350,13 @@ __global__ void __launch_bounds__(TK_THREADS) search_tail_kernel(const SearchArg
   __shared__ unsigned long long s_red[32];
   __shared__ unsigned long long s_out[MAX_CAND];
   __shared__ float s_lse[MAX_BEAM];
+  __shared__ int s_ts_only[MAX_BEAM];
   __shared__ int s_pick[MAX_BEAM];
   __shared__ int s_best_k;
   __shared__ int s_finished;
   __shared__ int s_last;
   if (a.st->all_done) return;  // a step enqueued ahead of the host's poll: nothing left to do
-  topk_merge_body(a, s_red, s_out, s_lse);
+  topk_merge_body(a, s_red, s_out, s_lse, s_ts_only);
   __syncthreads();  // the candidate list (global) is complete for this CTA's readers
   if (threadIdx.x < 32) search_bookkeeping_body(a, s_pick, s_best_k, s_finished);
   __syncthreads();
@@ -381,6 +455,12 @@ void search_step_run(const SearchArgs& a, cudaStream_t stream) {
   const int R = a.n_utt * a.beam;
   WISB_REQUIRE(a.beam >= 1 && a.beam <= MAX_BEAM && a.n_cand <= MAX_CAND, "search: beam_size must be in [1, 8]");
   WISB_REQUIRE((a.n_vocab + TOPK_CHUNKS - 1) / TOPK_CHUNKS <= TK_THREADS * TK_PER, "search: vocabulary too large");
+  if (a.ts_begin >= 0) {
+    WISB_REQUIRE(a.ts_begin > a.eot && a.ts_begin < a.n_vocab, "search: the vocabulary has no timestamp tokens");
+    WISB_REQUIRE(a.max_init_ts >= 0 && a.max_init_ts < a.n_vocab - a.ts_begin, "search: max_initial_timestamp_index out of range");
+    WISB_REQUIRE(cdiv(a.ts_begin, TOPK_CHUNKS - 1) <= TK_THREADS * TK_PER && a.n_vocab - a.ts_begin <= TK_THREADS * TK_PER,
+                 "search: vocabulary too large for timestamp decoding");
+  }
   topk_partial_kernel<<<dim3(TOPK_CHUNKS, R), TK_THREADS, 0, stream>>>(a);
   search_tail_kernel<<<a.n_utt, TK_THREADS, 0, stream>>>(a);
   WISB_CUDA(cudaGetLastError());

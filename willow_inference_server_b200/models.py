@@ -155,7 +155,9 @@ class Whisper:
                  return_no_speech_prob: bool = False, max_initial_timestamp_index: int = 50,
                  suppress_blank: bool = True, suppress_tokens=(-1,), sampling_topk: int = 1,
                  sampling_temperature: float = 1):
-        """ctranslate2.models.Whisper.generate for the options WIS relies on (SURVEY.md section 8b defaults)."""
+        """ctranslate2.models.Whisper.generate for the options WIS relies on (SURVEY.md section 8b defaults).  As in
+        CTranslate2, prompts without <|notimestamps|> decode with Whisper's timestamp rules (``max_initial_timestamp_index``
+        bounds the first timestamp) and ``sequences_ids`` then contain the timestamp tokens."""
         mel = _features_array(features)
         n = mel.shape[0]
         if len(prompts) != n:
@@ -170,8 +172,15 @@ class Whisper:
                              "(the CTranslate2 defaults WIS uses) are implemented")
         if not suppress_blank or -1 not in suppress_tokens or asynchronous:
             raise ValueError("suppress_blank=True, suppress_tokens containing -1 and asynchronous=False are required")
-        if self._dims["no_timestamps"] not in prompts[0]:
-            raise ValueError("timestamp decoding is not implemented: the prompt must contain <|notimestamps|>")
+        # CTranslate2's switch: a prompt without <|notimestamps|> turns the timestamp rules on (main.py:529, :661)
+        no_ts = self._dims["no_timestamps"]
+        modes = {no_ts not in p for p in prompts}
+        if len(modes) != 1:
+            raise ValueError("all prompts of one call must agree on <|notimestamps|> (timestamp decoding or not)")
+        timestamps = modes.pop()
+        n_ts = self._dims["n_vocab"] - no_ts - 1  # timestamp tokens [no_timestamps + 1, n_vocab)
+        if timestamps and not 0 <= int(max_initial_timestamp_index) < n_ts:
+            raise ValueError(f"max_initial_timestamp_index must be in [0, {n_ts - 1}], got {max_initial_timestamp_index}")
         extra = [int(t) for t in suppress_tokens if t >= 0]
         p = np.asarray(prompts, np.int32)
         parts = self._split(n, mel)
@@ -181,9 +190,11 @@ class Whisper:
         if ml is not None and ml.shape != (n,):
             raise ValueError("max_length must be an int or one int per feature window")
 
+        ts_kw = {"timestamps": True, "max_initial_timestamp_index": int(max_initial_timestamp_index)} if timestamps else {}
+
         def job(i, s, e):
             return lambda: self._handles[i].generate(mel[s:e], p[s:e], beam_size, patience, length_penalty,
-                                                     max_length if ml is None else ml[s:e], extra)
+                                                     max_length if ml is None else ml[s:e], extra, **ts_kw)
 
         outs = self._run([job(*pt) for pt in parts])
         results = []

@@ -199,7 +199,8 @@ def pack_state_dict(sd: dict, dims: WhisperDims) -> dict:
 # seeded synthetic weights (there are no real checkpoints in this image)
 # ---------------------------------------------------------------------------
 def synth_state_dict(dims: WhisperDims, seed: int = 0, logit_std: float = 4.0, qk_gain: float = 2.5,
-                     resid_std: float = 8.0, eot_ramp: tuple | None = None, script: tuple | None = None) -> dict:
+                     resid_std: float = 8.0, eot_ramp: tuple | None = None, script: tuple | None = None,
+                     ts_script: tuple | None = None) -> dict:
     """Deterministic random Whisper weights under HF names.
 
     Every GEMM weight is rounded to float16 so oracle (fp32 math) and engine
@@ -218,8 +219,16 @@ def synth_state_dict(dims: WhisperDims, seed: int = 0, logit_std: float = 4.0, q
     candidates are separated by O(rho) deviations instead of the ~0.01-wide near-ties of a flat random model,
     so greedy / beam transcripts are robust to fp16-vs-fp32 rounding.  The share of the residual stream the
     script takes is solved from ``rho`` and d_model, so the same setting works at every model size.
+
+    ``ts_script=((pos, first), ...)`` (needs ``script``) makes a model that speaks in timestamps: at each listed decoder
+    position the ``n_alt`` plausible next tokens are the timestamps ``no_timestamps + 1 + first + [0, n_alt)`` instead of
+    text tokens.  The ranges must be disjoint and increase with the position (timestamps never decrease), and the first
+    one should lie within the ``max_initial_timestamp_index`` the model is decoded with.  ``None`` leaves the weights
+    byte-identical to a call without it.
     """
     dims.validate()
+    if ts_script is not None and script is None:
+        raise ValueError("ts_script needs script=(n_alt, rho, off)")
     d = dims.d_model
     # logits = LN(x) . E[v] ~ N(0, d * emb_std^2): pick emb_std for the requested logit spread, and
     # make the sub-layer outputs large enough (residual stream std ~ resid_std) that the direct
@@ -327,6 +336,16 @@ def synth_state_dict(dims: WhisperDims, seed: int = 0, logit_std: float = 4.0, q
         s_eff = resid_std / np.sqrt(1.0 - frac)  # residual-stream std once the scripted components are in it
         banned = set(dims.suppress_ids) | set(dims.suppress_ids_begin)
         rng = np.random.default_rng(np.random.SeedSequence(entropy=ss.entropy, spawn_key=(10 ** 6,)))
+        ts_alts = {}
+        if ts_script is not None:
+            ts_rng = np.random.default_rng(np.random.SeedSequence(entropy=ss.entropy, spawn_key=(10 ** 6 + 1,)))
+            ts_begin = dims.no_timestamps + 1
+            prev_end = 0
+            for p, first in sorted((int(p), int(f)) for p, f in ts_script):
+                if p in ts_alts or first < prev_end or ts_begin + first + int(n_alt) > dims.n_vocab:
+                    raise ValueError("ts_script: timestamp ranges must be disjoint, increasing and inside the vocabulary")
+                prev_end = first + int(n_alt)
+                ts_alts[p] = [ts_begin + first + int(j) for j in ts_rng.permutation(int(n_alt))]
         pos = sd[dd + "embed_positions.weight"].astype(np.float64)
         for p in range(dims.n_text_ctx):
             alts = []
@@ -334,6 +353,7 @@ def synth_state_dict(dims: WhisperDims, seed: int = 0, logit_std: float = 4.0, q
                 t = int(rng.integers(300, dims.eot))  # ordinary text tokens only
                 if t not in banned and t not in alts:
                     alts.append(t)
+            alts = ts_alts.get(p, alts)  # (the text draw above still happens: later positions keep their tokens)
             for j, t in enumerate(alts):
                 nrm = np.linalg.norm(emb[t])
                 pos[p] += (c[j] * s_eff * logit_std / (nrm * nrm)) * emb[t].astype(np.float64)
